@@ -2,7 +2,7 @@
 """bench.py — Mpixels/s of the full PostProcess chain (PostFX prep -> SSR -> SSAO -> compose -> TAA -> Bloom -> ToneMap+sRGB)
 on a synthetic 3840x2160 G-buffer (BASELINE.json metric / configs[2]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--width 3840 --height 2160]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--width 3840 --height 2160] [--dump-outputs DIR]
 
 One "step" = one frame of the chain. Rank r (one process per GPU; torchrun for N > 1) processes its own sequence of
 frames: frames of a batch are independent sequences (SURVEY.md §8e, config 5: replicas, no data-path collective), so
@@ -168,6 +168,23 @@ class ClockSampler:
                 pass
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(smax) if smax else None, "reasons": sorted(reasons),
                 "samples": len(sm)}
+
+
+DUMP_PIXELS = 1 << 21   # 32 MB of RGBA float32
+
+
+def dump_outputs(out_dir: str, ldr) -> None:
+    """Writes what the timed path returned in its last step - the LDR plane of PostProcessChain.execute, RGBA float32 - as
+    out_dir/ldr.npy with one row per pixel: the whole frame in raster order when it has at most DUMP_PIXELS pixels, else a fixed,
+    seeded sample of DUMP_PIXELS of them (ascending raster index). The same --width / --height give the same pixels, so the
+    files of two builds compare output for output."""
+    import numpy as np
+    import torch
+    n = ldr.shape[0] * ldr.shape[1]
+    idx = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    rows = ldr.reshape(n, 4)[torch.from_numpy(idx).to(ldr.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "ldr.npy"), rows.astype(np.float32))
 
 
 def cpu_baseline(width: int, height: int, frames: int, threads: int) -> dict:
@@ -452,6 +469,8 @@ def main() -> None:
                     help="device-resident arm: G-buffer planes in the renderer's formats (RGBA16F / RG16F / RG8, what the passes read directly) or widened to fp32")
     ap.add_argument("--no-graph", action="store_true", help="issue every frame eagerly (no CUDA-graph replay)")
     ap.add_argument("--dof", action="store_true", help="add DepthOfField between TAA and Bloom (NOT the BASELINE.json workload; config.workload says so)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last one's LDR result to DIR/ldr.npy: RGBA float32, one row per pixel, "
+                         "a fixed seeded sample of 2^21 pixels of larger frames")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
@@ -579,6 +598,8 @@ def main() -> None:
     launches = lib.dfx_launch_count() - launches0
     issue = chain.stats()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, chain.ldr)   # before the legs below run more frames into the same plane
     ms_per_step = total_ms / K
     value = world * W * H / 1e6 / (ms_per_step / 1e3)
 

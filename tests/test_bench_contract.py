@@ -61,3 +61,48 @@ def test_reference_arm_live(built):
     if rec["cpu_baseline"]["kind"] == "reference":
         assert rec["value"] < rec["port"]["value"] * 1.5          # the checker-grade shader runner is not faster than the port by much, if at all
     assert rec["e2e"] == {"value": rec["value"], "unit": rec["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def _bench_module():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("dfx_bench", os.path.join(ROOT, "bench.py"))
+    m = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(m)
+    return m
+
+
+def test_dump_outputs_writes_a_fixed_sample_of_the_ldr_plane(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    bench = _bench_module()
+    ldr = torch.rand((30, 20, 4), generator=torch.Generator().manual_seed(1))
+    bench.dump_outputs(str(tmp_path / "whole"), ldr)
+    assert np.array_equal(np.load(tmp_path / "whole" / "ldr.npy"), ldr.numpy().reshape(-1, 4))   # small frames: every pixel, raster order
+    monkeypatch.setattr(bench, "DUMP_PIXELS", 100)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), ldr)
+    a, b = np.load(tmp_path / "a" / "ldr.npy"), np.load(tmp_path / "b" / "ldr.npy")
+    assert a.shape == (100, 4) and a.dtype == np.float32 and np.array_equal(a, b)
+    flat = ldr.numpy().reshape(-1, 4)
+    idx = [int(np.flatnonzero((flat == r).all(axis=1))[0]) for r in a]
+    assert idx == sorted(set(idx))                                                    # distinct pixels, ascending raster index
+
+
+@pytest.mark.gpu
+def test_steps_and_dumped_outputs(built, tmp_path):
+    """--steps is the number of timed frames (the kernel launches counted in the timed region grow with it in proportion), and
+    --dump-outputs writes the last timed frame's LDR plane, the same for the same arguments."""
+    import numpy as np
+
+    def run(steps: int, out) -> dict:
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "3", "--width", "320", "--height", "180",
+               "--no-cpu-baseline", "--no-psnr", "--dump-outputs", str(out)]
+        lines = subprocess.run(cmd, check=True, capture_output=True, text=True, timeout=600).stdout.strip().splitlines()
+        assert len(lines) == 1, lines
+        return json.loads(lines[0])
+
+    a, b, c = run(2, tmp_path / "a"), run(6, tmp_path / "b"), run(6, tmp_path / "c")
+    assert (a["steps"], b["steps"]) == (2, 6) and a["gpu_launches"] >= 40 and b["gpu_launches"] * 2 == a["gpu_launches"] * 6
+    ldr = np.load(tmp_path / "b" / "ldr.npy")
+    assert ldr.shape == (320 * 180, 4) and ldr.dtype == np.float32 and np.isfinite(ldr).all() and ldr[:, :3].max() > 0
+    assert np.array_equal(ldr, np.load(tmp_path / "c" / "ldr.npy"))

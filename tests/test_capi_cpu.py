@@ -29,11 +29,11 @@ def test_exports_every_declared_symbol(lib):
     assert r.returncode == 0, r.stderr
 
 
-def test_constant_block_sizes_match_reference_layout(lib):
+def test_constant_block_sizes_match_reference_layout(lib, tmp_path):
     # SURVEY.md §8a: 576 / 48 / 48 / 32 / 16 / 48 bytes
     src = '#include "dfx_b200.h"\n#include <stdio.h>\nint main(){printf("%zu %zu %zu %zu %zu %zu %zu\\n", sizeof(dfx_camera_attribs), sizeof(dfx_ssao_attribs),' \
           ' sizeof(dfx_ssr_attribs), sizeof(dfx_bloom_attribs), sizeof(dfx_taa_attribs), sizeof(dfx_tonemap_attribs), sizeof(dfx_plane));return 0;}'
-    exe = "/tmp/dfx_sizes_test"
+    exe = str(tmp_path / "dfx_sizes_test")
     subprocess.run(["gcc", "-x", "c", "-", "-I", os.path.dirname(capi.HEADER_PATH), "-o", exe], input=src.encode(), check=True)
     out = subprocess.check_output([exe]).decode().split()
     assert out[:6] == ["576", "48", "48", "32", "16", "48"]

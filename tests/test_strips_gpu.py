@@ -114,7 +114,7 @@ def test_two_gpus_bit_identical(built, tmp_path):
 
     from diligentfx_b200.strips import strip_bounds
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     if not torch.cuda.can_device_access_peer(0, 1):
         pytest.skip("GPUs 0 and 1 have no peer path")
     world = 2
