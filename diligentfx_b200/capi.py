@@ -25,6 +25,10 @@ SSR_FLAG_PREVIOUS_FRAME = 1
 POSTFX_FLAG_REVERSED_DEPTH = 1
 SSAO_FLAG_HALF_RESOLUTION = 2
 SSR_FLAG_HALF_RESOLUTION = 2
+# auto exposure (dfx_pass_update_average_luminance, dfx_chain_config.auto_exposure)
+AUTO_EXPOSURE_OFF, LUMINANCE_SAMPLING_REFERENCE, LUMINANCE_SAMPLING_FULL = 0, 1, 2
+AVERAGE_LUMINANCE_MAX_PARTIALS = 512
+AVERAGE_LUMINANCE_STATE_FLOATS = 8 + 2 * AVERAGE_LUMINANCE_MAX_PARTIALS   # [0] state, [1] max(0.05, state), [2] measurement, [3] its weight
 
 
 class Float4x4(C.Structure):
@@ -181,7 +185,7 @@ class ChainConfigC(C.Structure):
     _fields_ = [("ssao", SSAOAttribs), ("ssr", SSRAttribs), ("bloom", BloomAttribs), ("taa", TAAAttribs), ("tonemap", ToneMapAttribs), ("dof", DOFAttribs),
                 ("postfx_flags", C.c_uint32), ("ssao_flags", C.c_uint32), ("ssr_flags", C.c_uint32), ("taa_flags", C.c_uint32), ("dof_flags", C.c_uint32),
                 ("stages", C.c_uint32), ("enable_dof", C.c_int32), ("fuse", C.c_int32), ("overlap", C.c_int32), ("use_graph", C.c_int32), ("to_srgb", C.c_int32),
-                ("ave_log_lum", C.c_float), ("ssr_scale", C.c_float), ("ssao_scale", C.c_float), ("reserved", C.c_int32)]
+                ("ave_log_lum", C.c_float), ("ssr_scale", C.c_float), ("ssao_scale", C.c_float), ("auto_exposure", C.c_int32)]
 
 
 class ChainFrame(C.Structure):
@@ -228,6 +232,8 @@ def load(path: str = LIB_PATH) -> C.CDLL:
     lib.dfx_bloom_mip_count.restype = C.c_int32
     lib.dfx_chain_effect.restype = C.c_void_p
     lib.dfx_chain_post_stream.restype = C.c_void_p
+    lib.dfx_chain_average_luminance_dev.restype = C.c_void_p
+    lib.dfx_chain_set_elapsed_time.argtypes = [C.c_void_p, C.c_float]
     for name in declared_symbols():
         if not hasattr(lib, name):
             raise DfxError(f"libdfx_b200.so does not export {name}")

@@ -92,6 +92,9 @@ class ChainConfig:
     fuse: bool = True          # compose inside TAA, ToneMap inside the Bloom composite (same per-pixel arithmetic, two HBM round trips fewer)
     overlap: bool = True       # async compute: SSAO beside SSR on a second stream, Bloom + ToneMap beside the NEXT frame's front half on a third
     graph: bool = True         # replay steady-state frames from CUDA graphs (dfx_chain_config.use_graph)
+    # 0: tone-map with the constant ave_log_lum. capi.LUMINANCE_SAMPLING_REFERENCE (1) / _FULL (2): measure the scene's average luminance on
+    # the device and tone-map with the adapted value when tonemap.bAutoExposure is set (tonemap.bLightAdaptation + the elapsed time adapt it)
+    auto_exposure: int = 0
 
 
 class PostProcessChain:
@@ -130,6 +133,7 @@ class PostProcessChain:
         c.postfx_flags, c.ssao_flags, c.ssr_flags, c.taa_flags, c.dof_flags = cfg.postfx_flags, cfg.ssao_flags, cfg.ssr_flags, cfg.taa_flags, cfg.dof_flags
         c.stages, c.enable_dof, c.fuse, c.overlap, c.use_graph, c.to_srgb = cfg.stages, int(cfg.dof is not None), int(cfg.fuse), int(cfg.overlap), int(cfg.graph), int(cfg.to_srgb)
         c.ave_log_lum, c.ssr_scale, c.ssao_scale = cfg.ave_log_lum, cfg.ssr_scale, cfg.ssao_scale
+        c.auto_exposure = int(cfg.auto_exposure)
         return c
 
     def join(self):
@@ -164,14 +168,28 @@ class PostProcessChain:
         return n
 
     # ---- one frame ------------------------------------------------------------------------------------------------
+    def set_elapsed_time(self, seconds: float):
+        """Seconds since the previous frame (the reference's FrameAttribs.dElapsedTime) for light adaptation, from the next frame on."""
+        check(self.lib.dfx_chain_set_elapsed_time(self.chain, float(seconds)), "dfx_chain_set_elapsed_time")
+
+    def average_luminance(self) -> dict:
+        """The auto-exposure state after the frames issued so far (synchronises the device): the adapted luminance as the R16F target
+        holds it, the fAveLogLum the tone map used (max(0.05, state)), this frame's measurement exp(mean wlogL / mean w) and its weight."""
+        torch.cuda.synchronize(self.device)
+        out = download_plane(Plane(self.lib.dfx_chain_average_luminance_dev(self.chain), 16, 4, 1, capi.FORMAT_R32F, 0))[0]
+        return {"state": float(out[0]), "ave_log_lum": float(out[1]), "measured": float(out[2]), "weight": float(out[3])}
+
     def execute(self, frame_index: int, curr_camera, prev_camera, inputs: dict | None = None, ldr_out: torch.Tensor | None = None,
-                defer_post: bool = False) -> torch.Tensor:
+                defer_post: bool = False, elapsed_time: float | None = None) -> torch.Tensor:
         """Runs the chain on device-resident inputs (default: the planes filled by upload()); returns the final LDR plane
         (device tensor, rgba; `ldr_out` if given). Everything is ordered after the work already on the current stream. With
         cfg.overlap the LDR plane is produced on a side stream: by default the current stream waits for it before this call
         returns; `defer_post=True` skips that wait so that the next frame's front half overlaps it (call join() before
-        consuming the result)."""
+        consuming the result). `elapsed_time`: seconds since the previous frame for light adaptation (kept for later frames;
+        see set_elapsed_time)."""
         L, cfg = self.lib, self.cfg
+        if elapsed_time is not None:
+            self.set_elapsed_time(elapsed_time)
         c = self._config_struct()
         if bytes(c) != bytes(self._cfg_c):           # the caller edited self.cfg between frames
             self._cfg_c = c
@@ -192,7 +210,8 @@ class PostProcessChain:
         self.upload(frame)
         return self.execute(frame["frame"], frame["curr_camera"], frame["prev_camera"])
 
-    def stream_frames(self, frames, ldr_host: list | None = None, packed: bool = False, new_sequence: bool = False) -> int:
+    def stream_frames(self, frames, ldr_host: list | None = None, packed: bool = False, new_sequence: bool = False,
+                      elapsed_time: float | None = None) -> int:
         """Offline throughput path (BASELINE.json config 5: batches of frames): a double-buffered pipeline over three CUDA
         streams. While frame k runs on the compute stream, frame k+1's G-buffer is copied from (pinned) host memory on a
         copy stream and frame k-1's LDR result is copied back on a read-back stream; PCIe is full duplex, so the two copy
@@ -211,6 +230,8 @@ class PostProcessChain:
         first one), which stays on the device: in the reference the previous depth is last frame's depth target, not
         something the application uploads (HnPostProcessTask.cpp:788-832). Consecutive frames of one sequence then move 4 B/px less.
         The "frame streamed before" carries over from one call to the next unless `new_sequence=True`.
+
+        `elapsed_time`: seconds between frames for light adaptation (cfg.auto_exposure); a frame's own "elapsed_time" entry wins.
         """
         dev = self.device
         if not hasattr(self, "_pipe"):
@@ -259,7 +280,8 @@ class PostProcessChain:
             ins = P["inputs"][s]
             if packed:                                               # the passes read the render-target formats directly (Tex4 / Tex2 loaders): no widening pass
                 ins = {n: (P["staging"][s][n] if n in PACKED_SPECS else t) for n, t in P["inputs"][s].items()}
-            self.execute(fr["frame"], fr["curr_camera"], fr["prev_camera"], ins, ldr_out=P["ldr"][s], defer_post=True)
+            dt = fr.get("elapsed_time", elapsed_time)
+            self.execute(fr["frame"], fr["curr_camera"], fr["prev_camera"], ins, ldr_out=P["ldr"][s], defer_post=True, elapsed_time=dt)
             # the frame is complete when its Bloom + ToneMap (side stream under cfg.overlap) is: the event goes on that stream
             post = self._post_stream if self._side_post else main
             if post is not main:

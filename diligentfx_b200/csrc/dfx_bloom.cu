@@ -228,10 +228,11 @@ __global__ void __launch_bounds__(256) bloom_down2x_kernel(dfx_bloom_attribs A, 
 // (position x/2 - 1/4 resp. + 1/4 -> bilinear {1/4, 3/4}, convolved with the tent {1/4, 1/2, 1/4}). Clamp addressing is
 // applied when the 20x8 coarse tile is staged. COMPOSITE selects B4 (lerp with Intensity) instead of B3 (plain add).
 
-template <bool COMPOSITE, bool TONEMAP = false>
+template <bool COMPOSITE, bool TONEMAP = false, bool LUM_DEV = false>
 __global__ void __launch_bounds__(256) bloom_up2x_kernel(dfx_bloom_attribs A, View<const float4> fine, View<const float4> coarser, View<float4> out, int y0, int y1,
                                                          ToneMapIn tm = ToneMapIn{})
 {
+    if (LUM_DEV) tm.ave_log_lum = fmaxf(0.05f, __ldg(tm.ave_log_lum_dev)); // GetAverageSceneLuminance (AtmosphereShadersCommon.fxh:188-197)
     // A CTA of 256 threads produces 64x16 outputs; every thread a 2x2 block that shares one 5x5 coarse footprint, so the
     // shared-memory traffic is 25 LDS.128 per four outputs (the kernel would otherwise be bound by smem bandwidth, not HBM).
     __shared__ float4 tile[12][36];
@@ -455,10 +456,11 @@ __device__ __forceinline__ void up2x_stream_item(const dfx_bloom_attribs& A, con
     }
 }
 
-template <bool COMPOSITE, int TM>
+template <bool COMPOSITE, int TM, bool LUM_DEV = false>
 __global__ void __launch_bounds__(32 * kStreamWarps) bloom_up2x_stream_kernel(dfx_bloom_attribs A, View<const float4> fine, View<const float4> coarser, View<float4> out,
                                                                               int y0, int y1, int coarse_rows_per_warp, ToneMapIn tm)
 {
+    if (LUM_DEV) tm.ave_log_lum = fmaxf(0.05f, __ldg(tm.ave_log_lum_dev)); // GetAverageSceneLuminance (AtmosphereShadersCommon.fxh:188-197)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int fx0 = (blockIdx.x * kStreamWarps + warp) * 32;
     const int fyb = y0 + blockIdx.y * (2 * coarse_rows_per_warp), fye = min(fyb + 2 * coarse_rows_per_warp, y1); // y0 is even (checked by the caller)
@@ -759,11 +761,16 @@ static dfx_status launch_up(void* stream, int mode, const dfx_bloom_attribs& A, 
         // coarse rows per warp: dfx_tune("bloom_up_rows"), 0 = as few as fill one wave. Measured at 4K (profiles/r2i): 4 rows 0.062 ms for the
         // composite, 8 rows 0.064, 16 rows 0.066, one wave (25 rows) 0.070 - unlike the down-sampling, short warps win here.
         const int fixed_rows = dfx_tune_get("bloom_up_rows", 4);
+#define DFX_UP_LAUNCH_(COMP, TMODE, LD)                                                                                                              \
+    do {                                                                                                                                             \
+        const int  cpw = fixed_rows > 0 ? fixed_rows : stream_rows_per_warp(bloom_up2x_stream_kernel<COMP, TMODE, LD>, bx * kStreamWarps, n, 1);     \
+        const dim3 grid(bx, div_up(n, cpw));                                                                                                         \
+        bloom_up2x_stream_kernel<COMP, TMODE, LD><<<grid, 32 * kStreamWarps, 0, s>>>(A, fine, lo, out, rows.y0, rows.y1, cpw, tm);                   \
+    } while (0)
 #define DFX_UP_LAUNCH(COMP, TMODE)                                                                                                                   \
     do {                                                                                                                                             \
-        const int  cpw = fixed_rows > 0 ? fixed_rows : stream_rows_per_warp(bloom_up2x_stream_kernel<COMP, TMODE>, bx * kStreamWarps, n, 1);         \
-        const dim3 grid(bx, div_up(n, cpw));                                                                                                         \
-        bloom_up2x_stream_kernel<COMP, TMODE><<<grid, 32 * kStreamWarps, 0, s>>>(A, fine, lo, out, rows.y0, rows.y1, cpw, tm);                       \
+        if (TMODE >= 0 && tm.ave_log_lum_dev) DFX_UP_LAUNCH_(COMP, TMODE, true);                                                                     \
+        else DFX_UP_LAUNCH_(COMP, TMODE, false);                                                                                                     \
     } while (0)
         if (mode == 0) DFX_UP_LAUNCH(false, -1);
         else if (mode == 1) DFX_UP_LAUNCH(true, -1);
@@ -784,13 +791,15 @@ static dfx_status launch_up(void* stream, int mode, const dfx_bloom_attribs& A, 
                 default: DFX_UP_LAUNCH(true, DFX_TONE_MAPPING_MODE_COMMERCE); break;
             }
 #undef DFX_UP_LAUNCH
+#undef DFX_UP_LAUNCH_
     }
     else if (exact && (impl == 0 || mode == 2))
     {
         const dim3 grid(div_up(out.w, 64), div_up(rows.y1 - rows.y0, 16)), block(32, 8);
         if (mode == 0) bloom_up2x_kernel<false><<<grid, block, 0, s>>>(A, fine, lo, out, rows.y0, rows.y1);
         if (mode == 1) bloom_up2x_kernel<true><<<grid, block, 0, s>>>(A, fine, lo, out, rows.y0, rows.y1);
-        if (mode == 2) bloom_up2x_kernel<true, true><<<grid, block, 0, s>>>(A, fine, lo, out, rows.y0, rows.y1, tm);
+        if (mode == 2 && !tm.ave_log_lum_dev) bloom_up2x_kernel<true, true><<<grid, block, 0, s>>>(A, fine, lo, out, rows.y0, rows.y1, tm);
+        if (mode == 2 && tm.ave_log_lum_dev) bloom_up2x_kernel<true, true, true><<<grid, block, 0, s>>>(A, fine, lo, out, rows.y0, rows.y1, tm);
     }
     else
     {
@@ -844,6 +853,23 @@ extern "C" dfx_status dfx_pass_bloom_composite_tonemap(void* stream, const dfx_b
     DFX_REQUIRE(tonemap->iToneMappingMode >= 0 && tonemap->iToneMappingMode <= DFX_TONE_MAPPING_MODE_COMMERCE, "unknown tone mapping mode %d", tonemap->iToneMappingMode);
     if (rows.y1 == rows.y0) return DFX_OK;
     return launch_up(stream, 2, *attribs, c, u, out, rows, ToneMapIn{*tonemap, ave_log_lum, convert_to_srgb});
+}
+
+// the same with fAveLogLum = max(0.05, *ave_log_lum_dev), read by the kernel (the average-luminance state of dfx_exposure.cu)
+extern "C" dfx_status dfx_pass_bloom_composite_tonemap_dev(void* stream, const dfx_bloom_attribs* attribs, const dfx_tonemap_attribs* tonemap,
+                                                           const float* ave_log_lum_dev, int32_t convert_to_srgb, const dfx_plane* color, const dfx_plane* up0,
+                                                           const dfx_plane* ldr_out, dfx_rows rows)
+{
+    DFX_PROFILE(stream, "bloom_composite_tonemap");
+    DFX_REQUIRE(attribs && tonemap && ave_log_lum_dev, "null argument");
+    DFX_VIEW(const float4, c, color, DFX_FORMAT_RGBA32F);
+    DFX_VIEW(const float4, u, up0, DFX_FORMAT_RGBA32F);
+    DFX_VIEW(float4, out, ldr_out, DFX_FORMAT_RGBA32F);
+    DFX_SAME_SIZE(c, out);
+    DFX_REQUIRE(rows_ok(rows, out.h), "bad row range");
+    DFX_REQUIRE(tonemap->iToneMappingMode >= 0 && tonemap->iToneMappingMode <= DFX_TONE_MAPPING_MODE_COMMERCE, "unknown tone mapping mode %d", tonemap->iToneMappingMode);
+    if (rows.y1 == rows.y0) return DFX_OK;
+    return launch_up(stream, 2, *attribs, c, u, out, rows, ToneMapIn{*tonemap, 0.0f, convert_to_srgb, ave_log_lum_dev});
 }
 
 // First level the tail kernel takes over: the first one with at most kTailTexels texels (never level 0: it needs a source level).

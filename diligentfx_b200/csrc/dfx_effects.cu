@@ -63,8 +63,8 @@ struct dfx_postfx
     uint32_t            flags    = 0;
     bool                prepared = false, executed = false;
     uint8_t*            tables_dev = nullptr;
-    dfx_camera_attribs* cams_dev   = nullptr; // {curr, prev} followed by the frame index (uint32) the blue-noise pass reads
-    uint32_t*           frame_dev  = nullptr;
+    dfx_camera_attribs* cams_dev   = nullptr; // {curr, prev} followed by the frame index (uint32) the blue-noise pass reads and,
+    uint32_t*           frame_dev  = nullptr; // in the two words after it, the chain's elapsed time per ping-pong parity (float)
     PlaneOwner          bn_xy, bn_zw, reproj, prev_depth, closest;
     int                 w = 0, h = 0;
     ~dfx_postfx()
@@ -129,6 +129,10 @@ namespace dfx
 dfx_status launch_blue_noise(void* stream, const uint8_t* tables, uint32_t frame_index, const uint32_t* frame_index_dev, const dfx_plane* xy, const dfx_plane* zw);
 dfx_status launch_upload_cameras(void* stream, const dfx_camera_attribs* curr, const dfx_camera_attribs* prev, uint32_t frame_index, dfx_camera_attribs* dst_cams,
                                  uint32_t* dst_frame);
+dfx_status launch_upload_cameras(void* stream, const dfx_camera_attribs* curr, const dfx_camera_attribs* prev, uint32_t frame_index, dfx_camera_attribs* dst_cams,
+                                 uint32_t* dst_frame, float elapsed, float* dst_elapsed);
+dfx_status launch_update_average_luminance(void* stream, int adapt, int32_t sampling, float dt, const float* dt_dev, const dfx_plane* color, float* state);
+dfx_status launch_reset_average_luminance(void* stream, float* state);
 }
 // upload {curr, prev} like the map-discard of PostFXContext.cpp:310-318, plus the frame index (as kernel parameters: dfx_postfx.cu)
 static dfx_status postfx_upload(dfx_postfx* c, cudaStream_t s, const dfx_camera_attribs* curr, const dfx_camera_attribs* prev)
@@ -548,7 +552,7 @@ extern "C" dfx_status dfx_bloom_prepare(dfx_bloom* fx, dfx_postfx* postfx, uint3
 }
 
 static dfx_status bloom_execute_impl(dfx_bloom* fx, const dfx_bloom_render_attribs* a, const dfx_tonemap_attribs* tonemap, float ave_log_lum,
-                                     int32_t to_srgb, const dfx_plane* ldr_out);
+                                     int32_t to_srgb, const dfx_plane* ldr_out, const float* ave_log_lum_dev = nullptr);
 
 extern "C" dfx_status dfx_bloom_execute(dfx_bloom* fx, const dfx_bloom_render_attribs* a) { return bloom_execute_impl(fx, a, nullptr, 0.0f, 0, nullptr); }
 
@@ -560,9 +564,16 @@ extern "C" dfx_status dfx_bloom_execute_tonemapped(dfx_bloom* fx, const dfx_bloo
     DFX_REQUIRE(tonemap && ldr_out, "tonemap attribs / output plane must not be null");
     return bloom_execute_impl(fx, a, tonemap, ave_log_lum, convert_to_srgb, ldr_out);
 }
+// the same with fAveLogLum = max(0.05, *ave_log_lum_dev) (auto exposure: the chain's average-luminance state)
+static dfx_status dfx_bloom_execute_tonemapped_dev(dfx_bloom* fx, const dfx_bloom_render_attribs* a, const dfx_tonemap_attribs* tonemap, const float* ave_log_lum_dev,
+                                                   int32_t convert_to_srgb, const dfx_plane* ldr_out)
+{
+    DFX_REQUIRE(tonemap && ldr_out && ave_log_lum_dev, "tonemap attribs / luminance / output plane must not be null");
+    return bloom_execute_impl(fx, a, tonemap, 0.0f, convert_to_srgb, ldr_out, ave_log_lum_dev);
+}
 
 static dfx_status bloom_execute_impl(dfx_bloom* fx, const dfx_bloom_render_attribs* a, const dfx_tonemap_attribs* tonemap, float ave_log_lum,
-                                     int32_t to_srgb, const dfx_plane* ldr_out)
+                                     int32_t to_srgb, const dfx_plane* ldr_out, const float* ave_log_lum_dev)
 {
     EffectRange nvtx_range("Bloom");
     DFX_REQUIRE(fx && a, "null argument");
@@ -603,9 +614,11 @@ static dfx_status bloom_execute_impl(dfx_bloom* fx, const dfx_bloom_render_attri
     {
         const dfx_plane& u0 = fx->up[0].p;
         if (fx->w == 2 * u0.width && fx->h == 2 * u0.height)
-            return dfx_pass_bloom_composite_tonemap(s, &A, tonemap, ave_log_lum, to_srgb, a->color, &u0, ldr_out, rows(fx->out.p));
+            return ave_log_lum_dev ? dfx_pass_bloom_composite_tonemap_dev(s, &A, tonemap, ave_log_lum_dev, to_srgb, a->color, &u0, ldr_out, rows(fx->out.p))
+                                   : dfx_pass_bloom_composite_tonemap(s, &A, tonemap, ave_log_lum, to_srgb, a->color, &u0, ldr_out, rows(fx->out.p));
         if ((st = dfx_pass_bloom_composite(s, &A, a->color, &u0, &fx->out.p, rows(fx->out.p))) != DFX_OK) return st;
-        return dfx_pass_tonemap(s, tonemap, ave_log_lum, to_srgb, &fx->out.p, ldr_out, rows(fx->out.p));
+        return ave_log_lum_dev ? dfx_pass_tonemap_dev(s, tonemap, ave_log_lum_dev, to_srgb, &fx->out.p, ldr_out, rows(fx->out.p))
+                               : dfx_pass_tonemap(s, tonemap, ave_log_lum, to_srgb, &fx->out.p, ldr_out, rows(fx->out.p));
     }
     return dfx_pass_bloom_composite(s, &A, a->color, &fx->up[0].p, &fx->out.p, rows(fx->out.p));
 }
@@ -898,6 +911,8 @@ struct dfx_chain
     cudaEvent_t      ev_fork = nullptr, ev_ao_done = nullptr, ev_front_done = nullptr, post_done[2] = {nullptr, nullptr};
     bool             post_pending[2] = {false, false};
     PlaneOwner       composed;
+    float*           lum_state = nullptr; // average-luminance state of auto exposure (DFX_AVERAGE_LUMINANCE_STATE_FLOATS, dfx_exposure.cu)
+    float            elapsed   = 0.0f;    // dfx_chain_set_elapsed_time
     uint32_t         last_frame = ~0u;
     bool             graphs_ok  = true;
     std::map<std::string, GraphPair> graphs;
@@ -921,6 +936,7 @@ struct dfx_chain
             if (e) cudaEventDestroy(e);
         for (cudaStream_t s : {ao_stream, post_stream, cap_stream})
             if (s) cudaStreamDestroy(s);
+        cudaFree(lum_state);
     }
 };
 
@@ -962,7 +978,10 @@ extern "C" dfx_status dfx_chain_create(int32_t width, int32_t height, const dfx_
         if (e == cudaSuccess) e = cudaStreamCreateWithFlags(s, cudaStreamNonBlocking);
     for (cudaEvent_t* ev : {&c->ev_fork, &c->ev_ao_done, &c->ev_front_done, &c->post_done[0], &c->post_done[1]})
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&c->lum_state, DFX_AVERAGE_LUMINANCE_STATE_FLOATS * sizeof(float));
     if (st == DFX_OK && e != cudaSuccess) st = check_cuda(e, "dfx_chain_create");
+    if (st == DFX_OK) st = launch_reset_average_luminance(c->post_stream, c->lum_state);
+    if (st == DFX_OK && (e = cudaStreamSynchronize(c->post_stream)) != cudaSuccess) st = check_cuda(e, "dfx_chain_create");
     if (st != DFX_OK)
     {
         delete c;
@@ -1011,6 +1030,14 @@ extern "C" void* dfx_chain_effect(dfx_chain* c, int32_t which)
     }
 }
 extern "C" void* dfx_chain_post_stream(dfx_chain* c) { return c ? c->post_stream : nullptr; }
+extern "C" dfx_status dfx_chain_set_elapsed_time(dfx_chain* c, float seconds)
+{
+    DFX_REQUIRE(c, "null argument");
+    DFX_REQUIRE(seconds >= 0.0f && seconds < INFINITY, "elapsed time must be finite and >= 0 (got %g)", seconds);
+    c->elapsed = seconds;
+    return DFX_OK;
+}
+extern "C" const float* dfx_chain_average_luminance_dev(const dfx_chain* c) { return c ? c->lum_state : nullptr; }
 extern "C" dfx_status dfx_chain_get_stats(const dfx_chain* c, dfx_chain_stats* out)
 {
     DFX_REQUIRE(c && out, "null argument");
@@ -1035,6 +1062,7 @@ struct FrameCtx
     const dfx_chain_frame* f;
     uint32_t               st;
     bool                   side_ao, side_post, fuse_compose, fuse_tonemap, with_dof;
+    bool                   exposure, reset_lum; // auto exposure this frame; restart its state at 0.1 first (histories reset)
 };
 
 // PostFX .. TAA [.. DoF] on `s` (the SSAO passes fork to the chain's second stream and join before the compose). `*color_out` = what Bloom reads.
@@ -1109,13 +1137,24 @@ dfx_status record_post(const FrameCtx& x, cudaStream_t s, dfx_plane color)
     dfx_chain*              c   = x.c;
     const dfx_chain_config& cfg = c->cfg;
     dfx_status              st;
+    if (x.exposure)
+    {
+        // the scene luminance of the plane Bloom receives, measured and adapted before the composite reads it (EpipolarLightScattering.cpp:
+        // 2463-2481); the elapsed time is the word of this frame's parity that the camera upload wrote
+        if (x.reset_lum && (st = launch_reset_average_luminance(s, c->lum_state)) != DFX_OK) return st;
+        const float* dt_dev = reinterpret_cast<const float*>(c->pfx->frame_dev) + 1 + (x.f->frame_index & 1u);
+        if ((st = launch_update_average_luminance(s, cfg.tonemap.bLightAdaptation != 0, cfg.auto_exposure, 0.0f, dt_dev, &color, c->lum_state)) != DFX_OK) return st;
+    }
     if (x.st & DFX_CHAIN_STAGE_BLOOM)
     {
         dfx_bloom_render_attribs a{s, c->pfx, &color, &cfg.bloom};
+        if (x.fuse_tonemap && x.exposure) return dfx_bloom_execute_tonemapped_dev(c->bloom, &a, &cfg.tonemap, c->lum_state, cfg.to_srgb, x.f->ldr_out);
         if (x.fuse_tonemap) return dfx_bloom_execute_tonemapped(c->bloom, &a, &cfg.tonemap, cfg.ave_log_lum, cfg.to_srgb, x.f->ldr_out);
         if ((st = dfx_bloom_execute(c->bloom, &a)) != DFX_OK) return st;
         if ((st = dfx_bloom_get_plane(c->bloom, DFX_BLOOM_PLANE_OUTPUT, &color)) != DFX_OK) return st;
     }
+    if ((x.st & DFX_CHAIN_STAGE_TONEMAP) && x.exposure)
+        return dfx_pass_tonemap_dev(s, &cfg.tonemap, c->lum_state, cfg.to_srgb, &color, x.f->ldr_out, dfx_rows{0, c->h});
     if (x.st & DFX_CHAIN_STAGE_TONEMAP) return dfx_pass_tonemap(s, &cfg.tonemap, cfg.ave_log_lum, cfg.to_srgb, &color, x.f->ldr_out, dfx_rows{0, c->h});
     return DFX_OK;
 }
@@ -1133,7 +1172,12 @@ extern "C" dfx_status dfx_chain_execute(dfx_chain* c, void* stream, const dfx_ch
     const uint32_t          st  = cfg.stages;
     DFX_REQUIRE(!(st & (DFX_CHAIN_STAGE_TONEMAP)) || f->ldr_out, "the tone-mapped output plane must be given");
     cudaStream_t main = as_stream(stream);
-    FrameCtx     x{c, f, st, false, false, false, false, false};
+    FrameCtx     x{c, f, st, false, false, false, false, false, false, false};
+    DFX_REQUIRE(cfg.auto_exposure >= 0 && cfg.auto_exposure <= DFX_LUMINANCE_SAMPLING_FULL, "unknown auto_exposure mode %d", cfg.auto_exposure);
+    // auto exposure is opt-in: the default configuration carries the reference's bAutoExposure = TRUE, and the constant ave_log_lum
+    // stays what a chain computes unless auto_exposure asks for the measurement
+    x.exposure  = cfg.auto_exposure != 0 && cfg.tonemap.bAutoExposure != 0 && (st & DFX_CHAIN_STAGE_TONEMAP);
+    x.reset_lum = c->last_frame == ~0u || f->frame_index != c->last_frame + 1u; // the histories' reset rule (SURVEY.md §8b)
     x.with_dof     = cfg.enable_dof != 0;
     x.side_ao      = cfg.overlap && (st & DFX_CHAIN_STAGE_SSAO) && (st & DFX_CHAIN_STAGE_SSR);
     x.side_post    = cfg.overlap && (st & DFX_CHAIN_STAGE_BLOOM) && (st & DFX_CHAIN_STAGE_TAA) && !x.with_dof;
@@ -1179,7 +1223,12 @@ extern "C" dfx_status dfx_chain_execute(dfx_chain* c, void* stream, const dfx_ch
         c->post_pending[par] = false;
     }
     // ---- cameras + frame index -> device memory (kernel parameters, no copy engine; outside the recorded graphs: they change every frame)
-    if ((st & DFX_CHAIN_STAGE_POSTFX) && (s = launch_upload_cameras(main, f->curr_camera, f->prev_camera, f->frame_index, c->pfx->cams_dev, c->pfx->frame_dev)) != DFX_OK) return s;
+    // the elapsed time goes to the word of this frame's parity: Bloom + ToneMap of the previous frame may still read the other one
+    // on the chain's third stream (the wait on post_done[par] above orders the frame before last)
+    if (((st & DFX_CHAIN_STAGE_POSTFX) || x.exposure) &&
+        (s = launch_upload_cameras(main, f->curr_camera, f->prev_camera, f->frame_index, c->pfx->cams_dev, c->pfx->frame_dev, c->elapsed,
+                                   reinterpret_cast<float*>(c->pfx->frame_dev) + 1 + par)) != DFX_OK)
+        return s;
 
     dfx_plane color{};
     bool      replayed = false;

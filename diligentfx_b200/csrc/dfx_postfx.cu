@@ -120,23 +120,31 @@ struct CameraUpload
 {
     dfx_camera_attribs cams[2];
     uint32_t           frame;
+    float              elapsed; // seconds since the previous frame (light adaptation, dfx_exposure.cu)
 };
-__global__ void __launch_bounds__(320) upload_cameras_kernel(const __grid_constant__ CameraUpload u, uint32_t* __restrict__ dst_cams, uint32_t* __restrict__ dst_frame)
+__global__ void __launch_bounds__(320) upload_cameras_kernel(const __grid_constant__ CameraUpload u, uint32_t* __restrict__ dst_cams, uint32_t* __restrict__ dst_frame,
+                                                             float* __restrict__ dst_elapsed)
 {
     constexpr int  kWords = int(2 * sizeof(dfx_camera_attribs) / 4);
     const uint32_t* src   = reinterpret_cast<const uint32_t*>(&u);
     if (threadIdx.x < kWords) dst_cams[threadIdx.x] = src[threadIdx.x];
     if (threadIdx.x == 0 && dst_frame) *dst_frame = u.frame;
+    if (threadIdx.x == 0 && dst_elapsed) *dst_elapsed = u.elapsed;
+}
+dfx_status launch_upload_cameras(void* stream, const dfx_camera_attribs* curr, const dfx_camera_attribs* prev, uint32_t frame_index, dfx_camera_attribs* dst_cams,
+                                 uint32_t* dst_frame, float elapsed, float* dst_elapsed)
+{
+    static_assert(2 * sizeof(dfx_camera_attribs) / 4 <= 320, "one thread per word");
+    CameraUpload u;
+    u.cams[0] = *curr, u.cams[1] = *prev, u.frame = frame_index, u.elapsed = elapsed;
+    upload_cameras_kernel<<<1, 320, 0, as_stream(stream)>>>(u, reinterpret_cast<uint32_t*>(dst_cams), dst_frame, dst_elapsed);
+    DFX_LAUNCHED("upload_cameras_kernel");
+    return DFX_OK;
 }
 dfx_status launch_upload_cameras(void* stream, const dfx_camera_attribs* curr, const dfx_camera_attribs* prev, uint32_t frame_index, dfx_camera_attribs* dst_cams,
                                  uint32_t* dst_frame)
 {
-    static_assert(2 * sizeof(dfx_camera_attribs) / 4 <= 320, "one thread per word");
-    CameraUpload u;
-    u.cams[0] = *curr, u.cams[1] = *prev, u.frame = frame_index;
-    upload_cameras_kernel<<<1, 320, 0, as_stream(stream)>>>(u, reinterpret_cast<uint32_t*>(dst_cams), dst_frame);
-    DFX_LAUNCHED("upload_cameras_kernel");
-    return DFX_OK;
+    return launch_upload_cameras(stream, curr, prev, frame_index, dst_cams, dst_frame, 0.0f, nullptr);
 }
 
 void preload_postfx_kernels() // force the lazily-loaded kernels of this file in (see dfx_strips.cu)

@@ -249,6 +249,20 @@ __global__ void __launch_bounds__(256) tonemap_kernel(dfx_tonemap_attribs A, flo
     if (to_srgb) c = linear_to_srgb(c);
     st_cs(&out.at(x, y), f4(c, C.w));
 }
+// the same with fAveLogLum = max(0.05, *lum_dev) (GetAverageSceneLuminance, AtmosphereShadersCommon.fxh:188-197), read on the device
+template <int MODE>
+__global__ void __launch_bounds__(256) tonemap_dev_kernel(dfx_tonemap_attribs A, const float* lum_dev, int to_srgb, View<const float4> in, View<float4> out,
+                                                          int y0, int y1)
+{
+    const int x = blockIdx.x * blockDim.x + threadIdx.x;
+    const int y = y0 + blockIdx.y;
+    if (x >= out.w || y >= y1) return;
+    const float  aveLogLum = fmaxf(0.05f, __ldg(lum_dev));
+    const float4 C = __ldg(&in.at(x, y));
+    float3       c = tone_map<MODE>(xyz(C), A, aveLogLum);
+    if (to_srgb) c = linear_to_srgb(c);
+    st_cs(&out.at(x, y), f4(c, C.w));
+}
 
 } // namespace dfx
 
@@ -378,5 +392,39 @@ extern "C" dfx_status dfx_pass_tonemap(void* stream, const dfx_tonemap_attribs* 
     }
 #undef TM_LAUNCH
     DFX_LAUNCHED("tonemap_kernel");
+    return DFX_OK;
+}
+
+extern "C" dfx_status dfx_pass_tonemap_dev(void* stream, const dfx_tonemap_attribs* attribs, const float* ave_log_lum_dev, int32_t convert_to_srgb,
+                                           const dfx_plane* color, const dfx_plane* out_, dfx_rows rows)
+{
+    DFX_PROFILE(stream, "tonemap");
+    DFX_REQUIRE(attribs && ave_log_lum_dev, "null argument");
+    DFX_VIEW(const float4, c, color, DFX_FORMAT_RGBA32F);
+    DFX_VIEW(float4, out, out_, DFX_FORMAT_RGBA32F);
+    DFX_SAME_SIZE(c, out);
+    DFX_REQUIRE(rows_ok(rows, out.h), "bad row range");
+    DFX_REQUIRE(attribs->iToneMappingMode >= 0 && attribs->iToneMappingMode <= DFX_TONE_MAPPING_MODE_COMMERCE, "unknown tone mapping mode %d", attribs->iToneMappingMode);
+    if (rows.y1 == rows.y0) return DFX_OK;
+    dim3         block(256), grid(div_up(out.w, 256), rows.y1 - rows.y0);
+    cudaStream_t s = as_stream(stream);
+#define TM_LAUNCH(M) tonemap_dev_kernel<M><<<grid, block, 0, s>>>(*attribs, ave_log_lum_dev, convert_to_srgb, c, out, rows.y0, rows.y1)
+    switch (attribs->iToneMappingMode)
+    {
+        case DFX_TONE_MAPPING_MODE_NONE: TM_LAUNCH(DFX_TONE_MAPPING_MODE_NONE); break;
+        case DFX_TONE_MAPPING_MODE_EXP: TM_LAUNCH(DFX_TONE_MAPPING_MODE_EXP); break;
+        case DFX_TONE_MAPPING_MODE_REINHARD: TM_LAUNCH(DFX_TONE_MAPPING_MODE_REINHARD); break;
+        case DFX_TONE_MAPPING_MODE_REINHARD_MOD: TM_LAUNCH(DFX_TONE_MAPPING_MODE_REINHARD_MOD); break;
+        case DFX_TONE_MAPPING_MODE_UNCHARTED2: TM_LAUNCH(DFX_TONE_MAPPING_MODE_UNCHARTED2); break;
+        case DFX_TONE_MAPPING_MODE_FILMIC_ALU: TM_LAUNCH(DFX_TONE_MAPPING_MODE_FILMIC_ALU); break;
+        case DFX_TONE_MAPPING_MODE_LOGARITHMIC: TM_LAUNCH(DFX_TONE_MAPPING_MODE_LOGARITHMIC); break;
+        case DFX_TONE_MAPPING_MODE_ADAPTIVE_LOG: TM_LAUNCH(DFX_TONE_MAPPING_MODE_ADAPTIVE_LOG); break;
+        case DFX_TONE_MAPPING_MODE_AGX: TM_LAUNCH(DFX_TONE_MAPPING_MODE_AGX); break;
+        case DFX_TONE_MAPPING_MODE_AGX_CUSTOM: TM_LAUNCH(DFX_TONE_MAPPING_MODE_AGX_CUSTOM); break;
+        case DFX_TONE_MAPPING_MODE_PBR_NEUTRAL: TM_LAUNCH(DFX_TONE_MAPPING_MODE_PBR_NEUTRAL); break;
+        default: TM_LAUNCH(DFX_TONE_MAPPING_MODE_COMMERCE); break;
+    }
+#undef TM_LAUNCH
+    DFX_LAUNCHED("tonemap_dev_kernel");
     return DFX_OK;
 }

@@ -159,6 +159,7 @@ struct ToneMapIn // what the Bloom composite needs to apply the final ToneMap(+s
     dfx_tonemap_attribs attribs;
     float               ave_log_lum;
     int                 to_srgb;
+    const float*        ave_log_lum_dev = nullptr; // the *_dev entries: fAveLogLum = max(0.05, *ave_log_lum_dev) instead of ave_log_lum
 };
 
 } // namespace dfx

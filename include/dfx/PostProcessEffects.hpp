@@ -438,6 +438,69 @@ inline void ToneMap(IDeviceContext* pDeviceContext, ITextureView* pSrcColorSRV, 
                   "ToneMap");
 }
 
+// ToneMap() with fAveLogLum = max(0.05, *pAveLogLumDev) read on the device (GetAverageSceneLuminance, AtmosphereShadersCommon.fxh:188-197):
+// pass AverageLuminance::GetStateDev() below, or any device float the caller keeps.
+inline void ToneMap(IDeviceContext* pDeviceContext, ITextureView* pSrcColorSRV, ITextureView* pDstColorRTV, const HLSL::ToneMappingAttribs& Attribs,
+                    const float* pAveLogLumDev, bool ConvertOutputToSRGB)
+{
+    DFX_DEV_CHECK_ERR(pSrcColorSRV != nullptr && pDstColorRTV != nullptr && pAveLogLumDev != nullptr, "views and luminance must not be null");
+    if (!pSrcColorSRV || !pDstColorRTV || !pAveLogLumDev) return;
+    const dfx_plane* src = pSrcColorSRV->GetPlane();
+    detail::Check(dfx_pass_tonemap_dev(detail::StreamOf(pDeviceContext), &Attribs, pAveLogLumDev, ConvertOutputToSRGB ? 1 : 0, src, pDstColorRTV->GetPlane(),
+                                       dfx_rows{0, src ? src->height : 0}),
+                  "ToneMap");
+}
+
+// Auto exposure with light adaptation, the part of EpipolarLightScattering that ToneMappingAttribs::bAutoExposure / bLightAdaptation
+// switch on (EpipolarLightScattering.cpp:2463-2481, UpdateAverageLuminance.fx): owns the persistent average-luminance state (the 1x1
+// R16F target of the reference, cleared to 0.1) and updates it from a colour view once per frame. Update() measures when
+// Attribs.bAutoExposure is set and adapts over dElapsedTime (FrameAttribs.dElapsedTime) when Attribs.bLightAdaptation is set.
+class AverageLuminance
+{
+public:
+    enum SAMPLING : int32_t
+    {
+        SAMPLING_REFERENCE = DFX_LUMINANCE_SAMPLING_REFERENCE, // 64x64 point samples, half-rounded mip chain: the reference's numbers
+        SAMPLING_FULL      = DFX_LUMINANCE_SAMPLING_FULL       // every pixel (a small highlight cannot be missed)
+    };
+    explicit AverageLuminance(SAMPLING Sampling = SAMPLING_FULL) : m_Sampling(Sampling)
+    {
+        if (detail::Check(dfx_plane_alloc(DFX_AVERAGE_LUMINANCE_STATE_FLOATS, 1, DFX_FORMAT_R32F, &m_State), "AverageLuminance"))
+            Reset(nullptr);
+    }
+    ~AverageLuminance() { dfx_plane_free(&m_State); }
+    AverageLuminance(const AverageLuminance&)            = delete;
+    AverageLuminance& operator=(const AverageLuminance&) = delete;
+
+    void Reset(IDeviceContext* pDeviceContext)
+    {
+        detail::Check(dfx_pass_reset_average_luminance(detail::StreamOf(pDeviceContext), GetStateDev()), "AverageLuminance::Reset");
+    }
+    void Update(IDeviceContext* pDeviceContext, ITextureView* pColorSRV, const HLSL::ToneMappingAttribs& Attribs, double dElapsedTime)
+    {
+        DFX_DEV_CHECK_ERR(pColorSRV != nullptr, "pColorSRV must not be null");
+        if (!pColorSRV || !Attribs.bAutoExposure) return;
+        detail::Check(dfx_pass_update_average_luminance(detail::StreamOf(pDeviceContext), &Attribs, m_Sampling, static_cast<float>(dElapsedTime),
+                                                        pColorSRV->GetPlane(), GetStateDev()),
+                      "AverageLuminance::Update");
+    }
+    float* GetStateDev() const { return static_cast<float*>(m_State.ptr); }
+
+private:
+    SAMPLING  m_Sampling;
+    dfx_plane m_State{};
+};
+
+// ToneMap() with the adapted luminance of `Lum` when Attribs.bAutoExposure is set, with fAveLogLum otherwise.
+inline void ToneMap(IDeviceContext* pDeviceContext, ITextureView* pSrcColorSRV, ITextureView* pDstColorRTV, const HLSL::ToneMappingAttribs& Attribs,
+                    const AverageLuminance& Lum, float fAveLogLum, bool ConvertOutputToSRGB)
+{
+    if (Attribs.bAutoExposure)
+        ToneMap(pDeviceContext, pSrcColorSRV, pDstColorRTV, Attribs, static_cast<const float*>(Lum.GetStateDev()), ConvertOutputToSRGB);
+    else
+        ToneMap(pDeviceContext, pSrcColorSRV, pDstColorRTV, Attribs, fAveLogLum, ConvertOutputToSRGB);
+}
+
 // The compose step that sits between SSAO and TAA in the reference integration (reduced form, SURVEY.md §8f rank 1).
 inline void ComposeSSRAndSSAO(IDeviceContext* pDeviceContext, ITextureView* pColorSRV, ITextureView* pSSRRadianceSRV, ITextureView* pAmbientOcclusionSRV,
                               float SSRScale, float SSAOScale, ITextureView* pDstColorRTV)

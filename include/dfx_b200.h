@@ -548,6 +548,36 @@ DFX_API dfx_status dfx_pass_bloom_composite_tonemap(void* stream, const dfx_bloo
                                                     int32_t convert_to_srgb, const dfx_plane* color, const dfx_plane* up0, const dfx_plane* ldr_out,
                                                     dfx_rows rows);
 
+/* Auto exposure with light adaptation (ToneMappingAttribs.bAutoExposure / bLightAdaptation, ToneMappingStructures.fxh:37,41). The
+ * reference implements it in EpipolarLightScattering: a 64x64 RG16F target of GetWeightedLogLum (AtmosphereShadersCommon.fxh:199-205,
+ * UnwarpEpipolarScattering.fx:285-307, point samples), GenerateMips down to 1x1 (EpipolarLightScattering.cpp:2469, :2503),
+ * UpdateAverageLuminancePS (UpdateAverageLuminance.fx:12-29) alpha-blended into a persistent 1x1 R16F cleared to 0.1
+ * (…cpp:1823-1827, :885-905), and the consumer max(0.05, state) -> ToneMap() (GetAverageSceneLuminance, AtmosphereShadersCommon.fxh:188-197).
+ *
+ * The state is a device buffer of DFX_AVERAGE_LUMINANCE_STATE_FLOATS floats, 16-byte aligned, owned by the caller:
+ *   [0] the adapted luminance, rounded to half as the R16F target holds it     [1] max(0.05, [0]): the fAveLogLum the tone map uses
+ *   [2] this frame's measurement exp(mean wlogL / mean w) (fp32, not rounded)  [3] the blend weight it entered with
+ *   [4..] scratch of the full-frame mode (a ticket word and the per-CTA partials; left ready for the next launch).
+ * dfx_pass_reset_average_luminance must run once before the first update. One update at a time per buffer (stream order).        */
+#define DFX_LUMINANCE_SAMPLING_REFERENCE 1 /* 64x64 point samples, half-rounded mip chain: the reference bit for bit; one CTA         */
+#define DFX_LUMINANCE_SAMPLING_FULL      2 /* every pixel, fp32 per CTA, fp64 fixed-order total; deterministic                     */
+#define DFX_AVERAGE_LUMINANCE_MAX_PARTIALS 512
+#define DFX_AVERAGE_LUMINANCE_STATE_FLOATS (8 + 2 * DFX_AVERAGE_LUMINANCE_MAX_PARTIALS)
+/* Measures `color` (RGBA32F or RGBA16F, any size) and blends the measurement into the state: weight
+ * (1 - exp(-elapsed_seconds)) * saturate(mean w / 1e-3) with attribs->bLightAdaptation, saturate(mean w / 1e-3) without.
+ * Replaces the luminance branch of ApplyInscatteredRadiancePS, GenerateMips and UpdateAverageLuminancePS (EpipolarLightScattering.cpp:2463-2481). */
+DFX_API dfx_status dfx_pass_update_average_luminance(void* stream, const dfx_tonemap_attribs* attribs, int32_t sampling, float elapsed_seconds,
+                                                     const dfx_plane* color, float* state_dev);
+/* state := 0.1 as R16F holds it (0.0999755859375; the clear of EpipolarLightScattering.cpp:885-905), scratch words zeroed. */
+DFX_API dfx_status dfx_pass_reset_average_luminance(void* stream, float* state_dev);
+/* dfx_pass_tonemap / dfx_pass_bloom_composite_tonemap with fAveLogLum = max(0.05, *ave_log_lum_dev) read on the device (pass the state
+ * buffer itself): bit-identical to the scalar entries given max(0.05, that value).                                                   */
+DFX_API dfx_status dfx_pass_tonemap_dev(void* stream, const dfx_tonemap_attribs* attribs, const float* ave_log_lum_dev,
+                                        int32_t convert_to_srgb, const dfx_plane* color, const dfx_plane* out, dfx_rows rows);
+DFX_API dfx_status dfx_pass_bloom_composite_tonemap_dev(void* stream, const dfx_bloom_attribs* attribs, const dfx_tonemap_attribs* tonemap,
+                                                        const float* ave_log_lum_dev, int32_t convert_to_srgb, const dfx_plane* color,
+                                                        const dfx_plane* up0, const dfx_plane* ldr_out, dfx_rows rows);
+
 /* Host-side pieces that the reference computes on the CPU. */
 /* TemporalAntiAliasing::GetJitterOffset (TemporalAntiAliasing.cpp:63-78, Halton(2,3) x16). */
 DFX_API void dfx_taa_jitter_offset(uint32_t frame_index, uint32_t width, uint32_t height, float out_jitter[2]);
@@ -804,7 +834,10 @@ typedef struct dfx_chain_config
     int32_t  to_srgb;     /* LinearToSRGB after the tone map (HnCopyFrame.psh:60-62)                                         */
     float    ave_log_lum; /* HnPostProcessTask.hpp:88                                                                        */
     float    ssr_scale, ssao_scale; /* compose: rgb += ssr.rgb * ssr.a * ssr_scale; rgb *= lerp(1, ao, ssao_scale)           */
-    int32_t  reserved;
+    /* 0: the constant ave_log_lum (HnCopyFrame.psh:35). 1 / 2 (DFX_LUMINANCE_SAMPLING_*): measure the colour Bloom receives and
+     * tone-map with the adapted luminance, when tonemap.bAutoExposure is set (else the constant); tonemap.bLightAdaptation and
+     * dfx_chain_set_elapsed_time drive the adaptation. The state restarts at 0.1 whenever the histories reset.               */
+    int32_t  auto_exposure;
 } dfx_chain_config;
 
 typedef struct dfx_chain_frame
@@ -847,6 +880,11 @@ DFX_API void*      dfx_chain_effect(dfx_chain* chain, int32_t which /* dfx_chain
 /* The stream Bloom + ToneMap run on when `overlap` is set (to order a read-back after a deferred frame). */
 DFX_API void*      dfx_chain_post_stream(dfx_chain* chain);
 DFX_API dfx_status dfx_chain_get_stats(const dfx_chain* chain, dfx_chain_stats* out);
+/* Seconds since the previous frame (FrameAttribs.dElapsedTime of the reference) for light adaptation, from the next dfx_chain_execute
+ * on; it travels with the cameras, so it may change every frame while frames keep replaying from graphs. Default 0. */
+DFX_API dfx_status dfx_chain_set_elapsed_time(dfx_chain* chain, float seconds);
+/* The chain's average-luminance state (layout above dfx_pass_update_average_luminance); valid in the post stream's order. */
+DFX_API const float* dfx_chain_average_luminance_dev(const dfx_chain* chain);
 
 /* ============================================================================================================ */
 /* 4. one frame split into row strips over the GPUs of a box (no reference counterpart)                          */

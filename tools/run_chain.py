@@ -25,6 +25,9 @@ ap.add_argument("--in", dest="src", metavar="DIR", help="directory of .npz frame
 ap.add_argument("--out", dest="dst", metavar="DIR", help="where the LDR frames go")
 ap.add_argument("--batch", type=int, default=8, help="frames in flight per stream_frames call (pinned host buffers for that many results)")
 ap.add_argument("--ppm", action="store_true", help="write binary PPM instead of .npy")
+ap.add_argument("--auto-exposure", choices=("off", "reference", "full"), default="off",
+                help="tone-map with the measured, adapted scene luminance: 64x64 samples as the reference takes them, or every pixel")
+ap.add_argument("--frame-time", type=float, default=1.0 / 60.0, metavar="S", help="seconds between frames, for light adaptation (default 1/60)")
 a = ap.parse_args()
 
 if a.write_synthetic:
@@ -34,7 +37,9 @@ if a.write_synthetic:
     print("wrote", a.frames, "frames to", a.write_synthetic)
     sys.exit(0)
 
-from diligentfx_b200.chain import PostProcessChain  # noqa: E402  (loads the CUDA library: fails loudly without it)
+from diligentfx_b200.chain import ChainConfig, PostProcessChain  # noqa: E402  (loads the CUDA library: fails loudly without it)
+
+config = ChainConfig(auto_exposure={"off": 0, "reference": 1, "full": 2}[a.auto_exposure])
 
 if a.src:
     if not a.dst:
@@ -45,12 +50,12 @@ if a.src:
         ap.error(f"no .npz frames in {a.src}")
     first = gbuffer_io.load_frame(paths[0])
     h, w = first["depth"].shape
-    chain = PostProcessChain(w, h)
+    chain = PostProcessChain(w, h, config)
     results = [torch.empty((h, w, 4), dtype=torch.uint8).pin_memory() for _ in range(a.batch)]
     done = 0
     for b0 in range(0, len(paths), a.batch):
         batch = [gbuffer_io.load_frame(p, pin=True) for p in paths[b0:b0 + a.batch]]
-        n = chain.stream_frames(batch, ldr_host=results, packed=True, new_sequence=(b0 == 0))
+        n = chain.stream_frames(batch, ldr_host=results, packed=True, new_sequence=(b0 == 0), elapsed_time=a.frame_time)
         torch.cuda.synchronize()
         for k in range(n):
             name = os.path.splitext(os.path.basename(paths[b0 + k]))[0] + (".ppm" if a.ppm else ".npy")
@@ -60,7 +65,8 @@ if a.src:
     print("done", done, "frames,", chain.lib.dfx_launch_count(), "launches")
 else:
     seq = synth.generate_sequence(a.width, a.height, a.frames)
-    chain = PostProcessChain(a.width, a.height)
+    chain = PostProcessChain(a.width, a.height, config)
+    chain.set_elapsed_time(a.frame_time)
     for fr in seq:
         chain.run_frame(fr)
     torch.cuda.synchronize()
